@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rows/s of scan + filter + hash-aggregate on the 100M-row Parca schema (BASELINE.json).
 
-  python bench.py --gpus N --steps K --warmup W [--impl frostgpu|reference]
+  python bench.py --gpus N --steps K --warmup W [--impl frostgpu|reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK / LOCAL_RANK / WORLD_SIZE).  A step is one execution of
 
@@ -23,12 +23,17 @@ bytes and roofline fraction.
          parts (host parse + H2D), executes, reads the result record back and drops the parts.
 `--impl reference` times the CPU restatement of the reference path (oracle/, a port: the Go
          engine cannot be built here) on all host cores, on a bounded sample of the same workload.
+`--dump-outputs DIR` writes the result record of the last timed step to DIR, one float64 .npy per
+         column (see dump_outputs).  The inputs are generated from a fixed seed, so two builds run
+         with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import hashlib
 import json
 import os
+import re
 import subprocess
 import sys
 import threading
@@ -93,6 +98,35 @@ def parity_of(gpu_rows: dict, ref_rows: dict) -> dict:
     return {"checked": True, "groups": len(ref_rows), "gpu_groups": len(gpu_rows), "mismatches": mism}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, rows: dict, key_names, agg_names) -> None:
+    """Writes a result ({key tuple: aggregate tuple}, as result_rows returns it) as out_dir/<column>.npy, float64, one file
+    per key column (by name, as in the key tuples) and per aggregate.  Rows are in key order (NULL last), so two runs
+    compare element for element whatever order the engine returned the groups in.  A string key is written as a 48-bit
+    BLAKE2b digest of its UTF-8 bytes (exact in float64), NULL as NaN.  A result of more than DUMP_BYTES keeps a fixed,
+    seeded sample of its rows."""
+    items = sorted(rows.items(), key=lambda kv: tuple((v is None, v) for _, v in kv[0]))
+    cap = DUMP_BYTES // (8 * max(1, len(key_names) + len(agg_names)))
+    if len(items) > cap:
+        keep = np.sort(np.random.default_rng(0).choice(len(items), cap, replace=False))
+        items = [items[i] for i in keep]
+
+    def num(v):
+        if v is None:
+            return np.nan
+        if isinstance(v, str):
+            return float(int.from_bytes(hashlib.blake2b(v.encode(), digest_size=6).digest(), "little"))
+        return float(v)
+
+    cols = {n: [num(k[j][1]) for k, _ in items] for j, n in enumerate(key_names)}
+    cols.update({n: [num(a[j]) for _, a in items] for j, n in enumerate(agg_names)})
+    os.makedirs(out_dir, exist_ok=True)
+    for n, vals in cols.items():
+        np.save(os.path.join(out_dir, re.sub(r"[^0-9A-Za-z.]+", "_", n).strip("_") + ".npy"), np.asarray(vals, dtype=np.float64))
+
+
 def oracle_rows(bufs, plan_scan, agg_names, threads, sample_rows=0, reps=1):
     """Runs the oracle over the given Parquet buffers; returns (result rows, best seconds, rows scanned)."""
     from oracle import oracle as orc
@@ -143,6 +177,7 @@ class ClockSampler(threading.Thread):
         if self.proc:
             try:
                 self.proc.terminate()
+                self.proc.wait(timeout=5)
             except Exception:
                 pass
 
@@ -193,12 +228,15 @@ def run_reference(args, rows_per_gpu):
     filt, aggs, groups = headline_query_exprs(0, rows_per_gpu)
     scan = GPUScan(None, TABLE, filt, _lib.PLAN_AGGREGATE, groups, aggs)
     plan, keep = scan._plan()
+    agg_names = [a.Name() for a in aggs]
     times, scanned = [], 0
     for it in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         res = table.execute(plan, threads=threads, max_rows=sample_rows)
         dt = time.perf_counter() - t0
         scanned = res.rows_scanned
+        if args.dump_outputs and it == args.warmup + args.steps - 1:
+            dump_outputs(args.dump_outputs, result_rows([res.to_batch(agg_names)]), sorted(g.Name() for g in groups), agg_names)
         res.close()
         if it >= args.warmup:
             times.append(dt)
@@ -326,7 +364,10 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="frostgpu", choices=["frostgpu", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step to DIR/<column>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rows_per_gpu = env_int("FROSTGPU_BENCH_ROWS", 100_000_000)
     if args.impl == "reference":
@@ -437,6 +478,8 @@ def main():
     total_rows = rows_per_gpu * world
     value = total_rows * args.steps / dt
     gpu_rows = result_rows(batches)  # the last timed step's record (at N > 1: the merged result, on every rank)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, gpu_rows, sorted(g.Name() for g in groups), agg_names)
 
     # ---- e2e: host Parquet buffers -> result record, every step --------------------------------------
     # The parts sit in page-locked host memory (where the Go side would have written them); a step

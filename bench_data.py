@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import hashlib
 import os
+import tempfile
 from concurrent.futures import ProcessPoolExecutor
 from typing import Dict, List, Tuple
 
@@ -109,9 +110,11 @@ def _write_part(args) -> Tuple[str, int]:
 
 
 def cache_dir(tag: str) -> str:
-    for base in ("/dev/shm", "/tmp"):
+    """Where generated parts are kept between runs: in memory (/dev/shm) if possible, else the temporary directory.
+    One directory per user, so that users sharing a machine never read or block each other's files."""
+    for base in ("/dev/shm", tempfile.gettempdir()):
         if os.path.isdir(base) and os.access(base, os.W_OK):
-            d = os.path.join(base, "frostgpu_bench", tag)
+            d = os.path.join(base, f"frostgpu_bench-{os.getuid()}", tag)
             os.makedirs(d, exist_ok=True)
             return d
     raise RuntimeError("no writable scratch directory")
